@@ -4,6 +4,7 @@ per-GPU batch 32 (= the reference's "total batch 256 on 8 GPUs", README.md:81-83
 ImageNet-shaped data, random-init weights.
 
     python bench.py --gpus 1 --steps 50 --warmup 5
+    python bench.py --gpus 1 --steps 50 --warmup 5 --dump-outputs DIR  # + one step's outputs as DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...   # the unmodified reference (unavailable offline: see DESIGN.md)
@@ -72,7 +73,16 @@ def parse():
     ap.add_argument("--extras-budget-s", type=float, default=240.0,
                     help="wall-clock budget of the extra sections; when it runs out the headline line is printed without them")
     ap.add_argument("--distill-steps", type=int, default=40)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed runs, reset the model to its seeded initial state, run the timed step (the "
+                         "captured graph) once on a seeded batch and write its loss, updated parameters and BatchNorm "
+                         "running statistics as DIR/<name>.npy, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "pure" or args.impl != "edl" or args.gpus != 1):
+        ap.error("--dump-outputs supports --mode pure --impl edl --gpus 1 only")
+    return args
 
 
 class ClockSampler:
@@ -346,6 +356,7 @@ def main():
                                  algo=args.algo, target_kind="probs",
                                  fused_optimizer=False if args.no_fused_opt else None,
                                  clip_norm=args.clip_norm or None)
+        initial = snapshot(trainer) if args.dump_outputs else None
 
     # synthetic host data (pinned): a small pool of distinct batches, cycled
     pool = 4
@@ -483,6 +494,12 @@ def main():
         sampler.end()
         clocks_note = "timed regions + identical untimed steps right after them (timed region < sampling period)"
     clocks = sampler.stop()
+    if args.dump_outputs:
+        restore(trainer, initial)
+        torch.manual_seed(4321)
+        x = torch.randn(B, 3, 224, 224).to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+        t = torch.softmax(torch.randn(B, 1000) * 2.0, -1).to(torch.bfloat16)
+        dump_outputs(args.dump_outputs, trainer.step(x, t, sync=True), trainer.model)
     clocks["window"] = clocks_note
 
     value = B * world * args.steps / (dev_ms / 1e3)
@@ -546,6 +563,45 @@ def main():
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+DUMP_PARAM_SAMPLE = 4 << 20  # float32 elements (16 MB): ResNet50_vd has 25.6 M parameters
+
+
+def snapshot(trainer):
+    """Copies of everything a training step changes: parameters, BatchNorm buffers, fp32 masters, momentum."""
+    model = {k: v.detach().clone() for k, v in trainer.model.state_dict().items()}
+    opt = trainer.opt.state_dict()
+    return model, {"lr": opt["lr"], "momentum": {k: v.clone() for k, v in opt["momentum"].items()},
+                   "master": {k: v.clone() for k, v in opt["master"].items()}}
+
+
+def restore(trainer, state):
+    """Copies ``snapshot()`` back in place, so that the captured step graph still points at the live tensors."""
+    import torch
+
+    with torch.no_grad():
+        trainer.model.load_state_dict(state[0])
+        trainer.opt.load_state_dict(state[1])
+
+
+def dump_outputs(out_dir, loss, model):
+    """What one training step hands its caller: the loss and the model it updated in place.  Writes ``loss.npy``,
+    ``params.npy`` (all parameters in ``named_parameters()`` order, or a fixed seeded sample of
+    ``DUMP_PARAM_SAMPLE`` of them, sorted by position) and ``bn_running_stats.npy`` (every floating-point buffer),
+    all float32."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    params = torch.cat([p.detach().float().flatten() for _, p in model.named_parameters()]).cpu().numpy()
+    if params.size > DUMP_PARAM_SAMPLE:
+        params = params[np.sort(np.random.default_rng(0).choice(params.size, DUMP_PARAM_SAMPLE, replace=False))]
+    bufs = [b.detach().float().flatten() for _, b in model.named_buffers() if b.is_floating_point()]
+    arrays = {"loss": loss.detach().float().reshape(1).cpu().numpy(), "params": params,
+              "bn_running_stats": torch.cat(bufs).cpu().numpy() if bufs else np.zeros(0, np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def allreduce_crosscheck(dp, dev, world):
