@@ -182,6 +182,60 @@ void adam_step(const c10::optional<Tensor>& param_lp, Tensor& master, Tensor& m,
                  (float)beta1, (float)beta2, (float)eps, (float)wd, decoupled, cur_stream());
 }
 
+// LARS / LAMB: `chunks` is the int64 [nchunks, 5] table of optim_layerwise.cu with offsets into these (window)
+// tensors, `partials` fp32 scratch of >= 2 * nchunks floats.  Every chunk start must be a multiple of 8 elements.
+bool check_layerwise(const c10::optional<Tensor>& param_lp, const Tensor& master, const Tensor& grad,
+                            const Tensor& chunks, const Tensor& partials, const Tensor& lr) {
+  check_f32(master, "master");
+  check_f32(partials, "partials");
+  check_f32(lr, "lr");
+  TORCH_CHECK(grad.is_cuda() && grad.is_contiguous(), "grad must be a contiguous CUDA tensor");
+  const bool gbf = grad.scalar_type() == at::kBFloat16;
+  TORCH_CHECK(gbf || grad.scalar_type() == at::kFloat, "grad must be bf16 or fp32");
+  TORCH_CHECK(grad.numel() == master.numel(), "grad / master size mismatch");
+  TORCH_CHECK(chunks.is_cuda() && chunks.scalar_type() == at::kLong && chunks.is_contiguous() && chunks.dim() == 2 &&
+                  chunks.size(1) == 5, "chunks must be a contiguous CUDA int64 [n, 5] table");
+  TORCH_CHECK(partials.numel() >= 2 * chunks.size(0), "partials too small");
+  TORCH_CHECK(reinterpret_cast<uintptr_t>(master.data_ptr()) % 16 == 0 &&
+                  reinterpret_cast<uintptr_t>(grad.data_ptr()) % 16 == 0, "master / grad must be 16-byte aligned");
+  if (param_lp.has_value() && param_lp->defined()) {
+    check_bf16(*param_lp, "param_lp");
+    TORCH_CHECK(param_lp->numel() == master.numel(), "param_lp / master size mismatch");
+    TORCH_CHECK(reinterpret_cast<uintptr_t>(param_lp->data_ptr()) % 16 == 0, "param_lp must be 16-byte aligned");
+  }
+  return gbf;
+}
+
+void lars_step(const c10::optional<Tensor>& param_lp, Tensor& master, Tensor& mom, const Tensor& grad,
+               const Tensor& chunks, Tensor& partials, const Tensor& lr, const c10::optional<Tensor>& grad_scale,
+               const c10::optional<Tensor>& found_inf, double momentum, double lars_coeff, double wd, double eps) {
+  const bool gbf = check_layerwise(param_lp, master, grad, chunks, partials, lr);
+  check_f32(mom, "mom");
+  TORCH_CHECK(mom.numel() == master.numel() && reinterpret_cast<uintptr_t>(mom.data_ptr()) % 16 == 0);
+  c10::cuda::CUDAGuard g(master.device());
+  edl::lars_step(opt_ptr<void>(param_lp), master.data_ptr<float>(), mom.data_ptr<float>(), grad.data_ptr(), gbf,
+                 chunks.data_ptr<int64_t>(), (int)chunks.size(0), partials.data_ptr<float>(), lr.data_ptr<float>(),
+                 opt_ptr<float>(grad_scale), opt_ptr<int>(found_inf), (float)momentum, (float)lars_coeff, (float)wd,
+                 (float)eps, cur_stream());
+}
+
+void lamb_step(const c10::optional<Tensor>& param_lp, Tensor& master, Tensor& m, Tensor& v, const Tensor& grad,
+               const Tensor& chunks, Tensor& partials, const Tensor& lr, const c10::optional<Tensor>& grad_scale,
+               const c10::optional<Tensor>& found_inf, const Tensor& step, double beta1, double beta2, double eps,
+               double wd) {
+  const bool gbf = check_layerwise(param_lp, master, grad, chunks, partials, lr);
+  check_f32(m, "m");
+  check_f32(v, "v");
+  check_f32(step, "step");
+  TORCH_CHECK(m.numel() == master.numel() && v.numel() == master.numel());
+  TORCH_CHECK(reinterpret_cast<uintptr_t>(m.data_ptr()) % 16 == 0 && reinterpret_cast<uintptr_t>(v.data_ptr()) % 16 == 0);
+  c10::cuda::CUDAGuard g(master.device());
+  edl::lamb_step(opt_ptr<void>(param_lp), master.data_ptr<float>(), m.data_ptr<float>(), v.data_ptr<float>(),
+                 grad.data_ptr(), gbf, chunks.data_ptr<int64_t>(), (int)chunks.size(0), partials.data_ptr<float>(),
+                 lr.data_ptr<float>(), opt_ptr<float>(grad_scale), opt_ptr<int>(found_inf), step.data_ptr<float>(),
+                 (float)beta1, (float)beta2, (float)eps, (float)wd, cur_stream());
+}
+
 // ------------------------------------------------------------------ losses
 void soft_ce_fwd(const Tensor& logits, const c10::optional<Tensor>& target,
                  const c10::optional<Tensor>& labels, Tensor& loss_out, Tensor& row_stats,
@@ -553,6 +607,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("bn_bwd_apply", &bn_bwd_apply);
   m.def("sgd_momentum", &sgd_momentum);
   m.def("adam_step", &adam_step);
+  m.def("lars_step", &lars_step);
+  m.def("lamb_step", &lamb_step);
   m.def("soft_ce_fwd", &soft_ce_fwd);
   m.def("soft_ce_bwd", &soft_ce_bwd);
   m.def("topk_acc", &topk_acc);

@@ -67,6 +67,17 @@ void adam_step(void* param_lp, float* master, float* m, float* v, const void* gr
                const int* found_inf, const float* step, float beta1, float beta2, float eps,
                float wd, bool decoupled, cudaStream_t stream);
 
+// ---- optim_layerwise.cu ----
+// LARS / LAMB over a chunk table (int64 [nchunks, 5]: start, len, first chunk of the entry, chunk count of the
+// entry, decay flag); partials: fp32 [nchunks, 2] scratch.  Two launches each (norm pass, update pass).
+void lars_step(void* param_lp, float* master, float* mom, const void* grad, bool grad_is_bf16,
+               const int64_t* chunks, int nchunks, float* partials, const float* lr, const float* grad_scale,
+               const int* found_inf, float momentum, float lars_coeff, float wd, float eps, cudaStream_t stream);
+void lamb_step(void* param_lp, float* master, float* m, float* v, const void* grad, bool grad_is_bf16,
+               const int64_t* chunks, int nchunks, float* partials, const float* lr, const float* grad_scale,
+               const int* found_inf, const float* step, float beta1, float beta2, float eps, float wd,
+               cudaStream_t stream);
+
 // sum(g^2) of a flat gradient buffer into *out (+=), and the global-norm clip factor
 //   grad_scale = min(1, max_norm / (sqrt(sum of parts) + 1e-6))   (parts: one squared-norm partial per rank)
 void grad_sqnorm(const void* grad, bool grad_is_bf16, int64_t n, float* out, cudaStream_t stream);

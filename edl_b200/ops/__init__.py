@@ -86,7 +86,7 @@ def reset_fallbacks() -> None:
 from .bn import batch_norm_act, BatchNormAct2d, scale_shift_act, bn_stats_into, set_fused_bn, drop_bn_hook  # noqa: E402
 from .loss import soft_cross_entropy, topk_accuracy  # noqa: E402
 from .pool import max_pool_3x3_s2, avg_pool_2x2, global_avg_pool  # noqa: E402
-from .optim import FlatSGDMomentum, FlatAdam  # noqa: E402
+from .optim import FlatSGDMomentum, FlatAdam, FlatLARS, FlatLAMB  # noqa: E402
 from .gemm import stem7_infer, stem7_supported  # noqa: E402
 from .gemm import (gemm_bf16, linear_bf16, conv1x1, conv_lib, conv3x3, conv3x3_supported, conv3x3_infer,  # noqa: E402
                    conv3x3_infer_supported, conv3x3_wgrad, conv3x3_wgrad_supported, conv3x3_s2, conv3x3_s2_infer,
@@ -98,7 +98,7 @@ __all__ = [
     "batch_norm_act", "BatchNormAct2d", "scale_shift_act", "bn_stats_into",
     "soft_cross_entropy", "topk_accuracy",
     "max_pool_3x3_s2", "avg_pool_2x2", "global_avg_pool",
-    "FlatSGDMomentum", "FlatAdam", "gemm_bf16", "linear_bf16", "conv1x1", "conv_lib", "conv3x3",
+    "FlatSGDMomentum", "FlatAdam", "FlatLARS", "FlatLAMB", "gemm_bf16", "linear_bf16", "conv1x1", "conv_lib", "conv3x3",
     "conv3x3_supported", "conv3x3_infer", "conv3x3_infer_supported", "stem7_infer", "stem7_supported",
     "conv3x3_wgrad", "conv3x3_wgrad_supported", "conv3x3_s2", "conv3x3_s2_infer", "conv3x3_s2_supported",
     "stem_conv", "stem_conv_supported", "conv3x3_pair", "conv3x3_pair_supported",

@@ -290,7 +290,8 @@ class ElasticDataParallel:
     # ------------------------------------------------------------------ optimizer inside the bucket hook
     def attach_optimizer(self, opt, fused: Optional[bool] = None):
         """Let the engine run ``opt`` (a ``FlatSGDMomentum`` on this engine's flat buffers) bucket by bucket: inside
-        the reduction kernel on > 1 rank, right behind the bucket's last gradient on one.  ``fused=None`` follows
+        the reduction kernel on > 1 rank, right behind the bucket's last gradient on one.  ``FlatLARS`` /
+        ``FlatLAMB`` run bucket by bucket on one rank only (``step_range``).  ``fused=None`` follows
         ``EDL_FUSED_OPT`` (default on).  Not used with loss scaling, clipping (both need every gradient before any
         update), the hierarchical or library reduction paths, or weight-decay masks on a single rank."""
         self.opt = opt
@@ -309,8 +310,12 @@ class ElasticDataParallel:
         was_sharded = self.state_sharded
         self.bucket_opt = False
         opt = self.opt
+        # per-tensor-norm optimizers (LARS, LAMB: ``step_range``) ride along on ONE rank only: a bucket holds whole
+        # tensors, so their update per bucket is exact; the fused multi-rank kernel is SGD-momentum's
+        layerwise = hasattr(opt, "step_range")
         ok = (opt is not None and getattr(self, "_want_bucket_opt", False) and self.device.type == "cuda"
-              and type(opt).__name__ == "FlatSGDMomentum" and opt.found_inf_is_comm_error()
+              and (type(opt).__name__ == "FlatSGDMomentum" or (layerwise and self.world == 1))
+              and opt.found_inf_is_comm_error()
               and opt.grad_scale_t is None and self.clip_norm is None and self.found_inf is None
               and not self.hier and (self.world == 1 or self.use_symm))
         if ok:
@@ -325,6 +330,9 @@ class ElasticDataParallel:
             self.bucket_opt = bool(self._fused_dtypes)
         for b in self.buckets:
             b.fused_opt = self.bucket_opt and b.dtype in self._fused_dtypes
+        if layerwise and self.bucket_opt:
+            # chunk tables of every bucket, uploaded now: never inside the captured step
+            opt.plan_ranges([(b.dtype, b.start, b.numel) for b in self.buckets if b.fused_opt])
         if self.bucket_opt and self.world > 1:
             if not self.param_slices:
                 self.flat.rebind_params(self._param_alloc, dtypes=self._fused_dtypes)
@@ -398,11 +406,17 @@ class ElasticDataParallel:
         rest of backward still runs (the separate whole-model optimizer pass at the end of the step disappears)."""
         from ..ops import native, count_launch
 
-        opt, st = self.opt, self.opt.state[b.dtype]
+        opt = self.opt
+        self._join_producers()
+        if hasattr(opt, "step_range"):                 # LARS / LAMB: norm pass + update pass over the bucket
+            with torch.cuda.stream(self.comm_stream):
+                opt.step_range(b.dtype, b.start, b.numel)
+            self.last_algos.append(("local_" + type(opt).__name__.lower(), b.numel * g.grad.element_size(), True))
+            return
+        st = opt.state[b.dtype]
         lo, hi = b.start, b.start + b.numel
         master = g.master if g.master is not None else g.param
         lp = g.param[lo:hi] if g.master is not None else None
-        self._join_producers()
         with torch.cuda.stream(self.comm_stream):
             native().sgd_momentum(lp, master[lo:hi], st["mom"][lo:hi], g.grad[lo:hi],
                                   st["wd_mask"][lo:hi] if st["wd_mask"] is not None else None, opt.lr_t, None,

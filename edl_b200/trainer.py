@@ -121,7 +121,7 @@ class StudentTrainer:
         # gradient first (loss scaling, clipping): fused reduce-scatter -> SGD -> all-gather kernel on > 1 GPU,
         # per-bucket optimizer launches on the side stream on one (parallel/ddp.py:attach_optimizer)
         self._fused_optimizer = fused_optimizer
-        if isinstance(self.opt, ops.FlatSGDMomentum):
+        if isinstance(self.opt, (ops.FlatSGDMomentum, ops.FlatLARS, ops.FlatLAMB)):
             self.dp.attach_optimizer(self.opt, fused=fused_optimizer)
         # recompute runs every block's forward twice: the pre-zeroed accumulate-into arena slices would
         # be summed twice, so those runs let each op allocate its own scratch

@@ -31,7 +31,8 @@ import edl_b200 as edl  # noqa: E402
 from edl_b200 import elastic, ops  # noqa: E402
 from edl_b200.checkpoint import LocalFS, TrainStatus, load_check_point, save_check_point  # noqa: E402
 from edl_b200.models import VGG, ResNet, ResNetVd, to_train_dtype  # noqa: E402
-from edl_b200.ops.optim import cosine_decay_with_warmup, piecewise_decay_with_warmup, scaled_lr  # noqa: E402
+from edl_b200.ops.optim import (cosine_decay_with_warmup, piecewise_decay_with_warmup,  # noqa: E402
+                                polynomial_decay_with_warmup, scaled_lr)
 from edl_b200.trainer import StudentTrainer  # noqa: E402
 from edl_b200.utils import train_status as edl_train_status  # noqa: E402
 from edl_b200.utils.metrics import StepMeter, write_benchmark_log  # noqa: E402
@@ -45,7 +46,13 @@ def parse():
     ap.add_argument("--batch_size", type=int, default=32, help="per trainer")
     ap.add_argument("--total_batch_size", type=int, default=0, help="if set, per-trainer batch = total / world")
     ap.add_argument("--lr", type=float, default=0.1)
-    ap.add_argument("--lr_strategy", default="cosine_decay_with_warmup", choices=["cosine_decay_with_warmup", "piecewise_decay"])
+    ap.add_argument("--lr_strategy", default="cosine_decay_with_warmup",
+                    choices=["cosine_decay_with_warmup", "piecewise_decay", "polynomial_decay"])
+    ap.add_argument("--optimizer", default="momentum", choices=["momentum", "lars", "lamb"],
+                    help="momentum SGD (the reference's default), LARS or LAMB (large global batches); LARS / LAMB "
+                         "leave 1-D parameters (BatchNorm scale / shift, biases) out of weight decay")
+    ap.add_argument("--lars_coeff", type=float, default=0.001)
+    ap.add_argument("--lars_weight_decay", type=float, default=5e-4)
     ap.add_argument("--steps_per_epoch", type=int, default=0, help="0 = total_images / (batch * world)")
     ap.add_argument("--total_images", type=int, default=1281167)
     ap.add_argument("--class_dim", type=int, default=1000)
@@ -89,6 +96,25 @@ def file_feed(args, bs, rank, world, epoch, skip, dev, dtype, cuda):
     return gen()
 
 
+def make_optimizer(args, lr):
+    """``StudentTrainer(optimizer=...)`` factory for ``--optimizer`` (None: the trainer's momentum SGD)."""
+    if args.optimizer == "momentum":
+        return None
+    no_decay = lambda name, p: p.dim() <= 1                  # noqa: E731  (BatchNorm scale / shift, biases)
+    if args.optimizer == "lars":
+        return lambda flat: ops.FlatLARS(flat, lr=lr, lars_coeff=args.lars_coeff,
+                                         lars_weight_decay=args.lars_weight_decay, exclude=no_decay)
+    return lambda flat: ops.FlatLAMB(flat, lr=lr, exclude=no_decay)
+
+
+def learning_rate(args, step, base_lr, steps_per_epoch):
+    if args.lr_strategy.startswith("cosine"):
+        return cosine_decay_with_warmup(step, base_lr, steps_per_epoch, args.epochs)
+    if args.lr_strategy == "polynomial_decay":
+        return polynomial_decay_with_warmup(step, base_lr, steps_per_epoch, args.epochs, warmup_epochs=5)
+    return piecewise_decay_with_warmup(step, base_lr, steps_per_epoch, [30, 60, 80])
+
+
 def main():
     args = parse()
     ctx = info = None
@@ -119,6 +145,7 @@ def main():
     tr = StudentTrainer(model, bs, image_shape=(3, args.image_size, args.image_size), num_classes=args.class_dim,
                         lr=base_lr, target_kind="labels", use_graph=cuda, dtype=dtype,
                         fabric=ctx.fabric if ctx is not None else None,   # GPUs in place: no process group at all
+                        optimizer=make_optimizer(args, base_lr),
                         loss_fn=lambda z, t: ops.soft_cross_entropy(z, t, "labels", label_smoothing=args.label_smoothing))
     fs = LocalFS()
 
@@ -159,8 +186,7 @@ def main():
         switch, failed = False, ""
         feed = file_feed(args, bs, rank, world, epoch, it, dev, dtype, cuda)
         while it < n_steps:
-            lr = (cosine_decay_with_warmup(step, base_lr, steps_per_epoch, args.epochs) if args.lr_strategy.startswith("cosine")
-                  else piecewise_decay_with_warmup(step, base_lr, steps_per_epoch, [30, 60, 80]))
+            lr = learning_rate(args, step, base_lr, steps_per_epoch)
             tr.set_lr(lr)
             if (ctx is not None and world > 1 and rank == 1 and not injected and args.inject_fault_file
                     and os.path.exists(args.inject_fault_file)):
